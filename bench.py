@@ -10,6 +10,9 @@ synthetic workload BASELINE.json's metric is quoted on: N=512 state, 600 feature
   N > 1 : one independent filter replica per GPU (the per-plane update chain does not shard, DESIGN.md §multi-GPU), weak scaling;
           the sharded large-update path (cfg5: 4000 features, NCCL all-gather of compressed [R z] blocks) is reported beside it
   --impl reference : the reference's CPU algorithm (oracle restatement, the reference cannot be compiled here) on the host cores
+  --dump-outputs DIR : the last `value` step's gates (feat_status, feat_chi2, plane_status, plane_chi2, hx_order) and posterior
+          state (x: variable values in State::_variables order, P) as DIR/<name>.npy in float64, about 2 MB (rank 0);
+          feat_chi2 / plane_chi2 hold only the individually gated features (feat_status 0, 1) / visited planes (plane_status 0, 1)
 """
 import argparse
 import json
@@ -200,7 +203,11 @@ def main():
     ap.add_argument("--impl", default="ours")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sharded", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed (gates and posterior x, P) "
+                                                          "as DIR/<name>.npy, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -283,7 +290,15 @@ def main():
         ev[k][1].record(stream)
     barrier()
     launches = ctx.launch_count() - l0
-    ctx.msckf_finish()
+    gates = ctx.msckf_finish()
+    if args.dump_outputs:  # read back now: the passes below restore and update the same filter again
+        # the ABI reports chi2 = NaN for features consumed by a plane update (status 2) and planes not visited (status -1):
+        # keep the chi2 of the gated entries only, selected by status so that a NaN from a gated entry still shows
+        gates["feat_chi2"] = gates["feat_chi2"][gates["feat_status"] != 2]
+        gates["plane_chi2"] = gates["plane_chi2"][gates["plane_status"] != -1]
+        dumped = {k: np.asarray(v, dtype=np.float64) for k, v in gates.items()}
+        dumped["x"] = np.concatenate([ctx.var_get(h)[0] for h in ctx.variable_order()])
+        dumped["P"] = ctx.cov()
     step_ms = [a.elapsed_time(b) for a, b in ev]
     per_rank_ms = gather_over_ranks(float(np.mean(step_ms)))
     ms_per_step = max_over_ranks(float(np.mean(step_ms)))
@@ -545,6 +560,10 @@ def main():
 
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         line["cpu_baseline"] = cpu_baseline_single()
+    if rank == 0 and args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for k, v in dumped.items():
+            np.save(os.path.join(args.dump_outputs, k + ".npy"), v)
     if rank == 0:
         print(json.dumps(line))
     ctx.close()
